@@ -39,6 +39,10 @@ NB = 8192                     # 16 GiB paged cache (BASELINE.md §3)
 SESSIONS, CTX = 16, 2048      # one wave of the 2K-ctx multi-round-QA config
 TOKEN_BYTES_ALL = 2 * L * H * D * 2   # 131072 B payload per token (bf16)
 ALGO_BYTES_PER_TOKEN = 2 * TOKEN_BYTES_ALL  # HBM read + HBM write of the gather kernel
+# --dump-outputs: a fixed, seeded sample of what each timed leg computed in its last step (~40 MiB in all)
+DUMP_TOKENS = 32              # tokens of the wave whose K and V rows in every layer are written
+DUMP_CHUNK_VALUES = 1 << 20   # values of the device leg's chunk buffer
+DUMP_LIMIT_BYTES = 64 * 10**6
 
 
 def peaks():
@@ -223,8 +227,6 @@ def run_ours(args):
     import torch
     import torch.distributed as dist
 
-    import __graft_entry__ as ge
-    ge.build(quiet=True)
     from b200kv import FMT_FP8, FMT_Q4, FMT_RAW, KVEngine, KVGeometry, KVPool
 
     rank = int(os.environ.get("RANK", "0"))
@@ -281,21 +283,38 @@ def run_ours(args):
     all_dst = np.concatenate(dst_maps)
     stream = torch.cuda.current_stream()
 
+    dumps = {}   # name -> array: what the timed legs computed in their last step (rank 0, --dump-outputs)
+    dumping = bool(args.dump_outputs) and rank == 0
+    if dumping:
+        dump_slots = torch.as_tensor(np.sort(all_dst[np.random.default_rng(7).choice(len(all_dst), DUMP_TOKENS, replace=False)]),
+                                     device=dev)
+        dst_blocks = torch.as_tensor(dperm[:SESSIONS * nblk].copy(), device=dev)
+
+    def dump_pages(leg, masks=None):
+        """The pages the last step wrote into (every session's destination blocks): K and V of DUMP_TOKENS
+        seeded tokens in every layer, a float64 sum per (layer, K|V, block) over all of them, and the
+        retrieve masks the caller was given."""
+        if masks is not None:
+            dumps[f"{leg}_ret_mask"] = masks.astype(np.float32)
+        dumps[f"{leg}_kv_rows"] = torch.stack([c.view(2, NB * BS, H, D)[:, dump_slots] for c in caches]).float().cpu().numpy()
+        dumps[f"{leg}_block_sums"] = torch.stack([c.view(2, NB, -1)[:, dst_blocks].double().sum(-1)
+                                                  for c in caches]).cpu().numpy()
+
     # ---- e2e leg: store + retrieve through the engine, host pool in the loop ------------------
     def e2e_step(step):
         # every session is stored, and retrieved as soon as ITS store has been committed to the
         # host index; retrieves of early sessions overlap the D2H of later ones (PCIe is full duplex)
         toks = [session_tokens(rank, step, s) for s in range(SESSIONS)]
         tickets = [eng.store(toks[s], None, src_maps[s], stream=stream) for s in range(SESSIONS)]
-        n = 0
+        masks = []
         for s in range(SESSIONS):
             eng.wait(tickets[s])
-            n += int(eng.retrieve(toks[s], None, dst_maps[s], stream=stream).sum())
-        return n
+            masks.append(eng.retrieve(toks[s], None, dst_maps[s], stream=stream))
+        return np.stack(masks)
 
     sampler = ClockSampler(local) if rank == 0 else None   # nvidia-smi needs ~1 s to start emitting
     for w in range(args.warmup):
-        assert e2e_step(w) == SESSIONS * CTX
+        assert e2e_step(w).sum() == SESSIONS * CTX
     torch.cuda.synchronize()
     st0 = eng.stats()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -303,12 +322,14 @@ def run_ours(args):
     ev0.record(stream)
     for k in range(args.steps):
         got = e2e_step(args.warmup + k)
-        assert got == SESSIONS * CTX, got
+        assert got.sum() == SESSIONS * CTX, got.sum()
     eng.wait_all()
     ev1.record(stream)
     torch.cuda.synchronize()
     barrier()
     my_e2e_ms = ev0.elapsed_time(ev1) / args.steps
+    if dumping:
+        dump_pages("e2e", got)
     e2e_ms = max_over_ranks(my_e2e_ms)
     st1 = eng.stats()
     e2e_payload = 2 * SESSIONS * CTX * TOKEN_BYTES_ALL
@@ -339,6 +360,12 @@ def run_ours(args):
     barrier()
     dev_ms = max_over_ranks(ev0.elapsed_time(ev1)) / args.steps
     st3 = eng.stats()
+    if dumping:
+        vals = dbuf.view(torch.bfloat16)
+        pick = np.sort(np.random.default_rng(8).integers(0, vals.numel(), DUMP_CHUNK_VALUES))
+        dumps["dev_chunks_sample"] = vals[torch.as_tensor(pick, device=dev)].float().cpu().numpy()
+        dumps["dev_chunk_sums"] = np.array([float(x.double().sum()) for x in vals.view(n_chunks_step, -1)])
+        dump_pages("dev")
     clocks = sampler.stop() if sampler else None
     value_gbps = world * e2e_payload / (dev_ms * 1e-3) / 1e9
     g_ms = float(np.mean([a for a, _ in gather_ms]))
@@ -445,7 +472,7 @@ def run_ours(args):
     pool.close()
 
     # ---- compressed-format legs (extra, not the headline): the same wave in FP8 and Q4 ------------
-    def format_leg(fmt, salt):
+    def format_leg(fmt, salt, leg):
         gq = KVGeometry(L, H, D, NB, BS, C, 2, 0, fmt)
         poolq = KVPool(None, (n_chunks_step + n_chunks_step // 2) * gq.chunk_bytes, gq.chunk_bytes, 1)
         eq = KVEngine(gq, poolq, local, staging_bytes=2 * n_chunks_step * gq.chunk_bytes, owner=rank)
@@ -455,9 +482,11 @@ def run_ours(args):
         def q_e2e(step):
             toks = [session_tokens(rank, salt + step, s_) for s_ in range(SESSIONS)]
             tickets = [eq.store(toks[s_], None, src_maps[s_], stream=stream) for s_ in range(SESSIONS)]
+            masks = []
             for s_ in range(SESSIONS):
                 eq.wait(tickets[s_])
-                eq.retrieve(toks[s_], None, dst_maps[s_], stream=stream)
+                masks.append(eq.retrieve(toks[s_], None, dst_maps[s_], stream=stream))
+            return np.stack(masks)
 
         for w in range(max(args.warmup, 1)):
             q_e2e(w)
@@ -466,12 +495,14 @@ def run_ours(args):
         barrier()
         ev0.record(stream)
         for k in range(args.steps):
-            q_e2e(args.warmup + k)
+            masks = q_e2e(args.warmup + k)
         eq.wait_all()
         ev1.record(stream)
         torch.cuda.synchronize()
         barrier()
         q_ms = max_over_ranks(ev0.elapsed_time(ev1)) / args.steps
+        if dumping:
+            dump_pages(leg, masks)
         km = []
         for k in range(args.steps):
             eq.gather(all_src, bq.data_ptr(), stream)
@@ -492,9 +523,9 @@ def run_ours(args):
 
     fp8 = q4 = None
     if not args.no_fp8:
-        fp8 = format_leg(FMT_FP8, 1000)
+        fp8 = format_leg(FMT_FP8, 1000, "fp8")
         try:
-            q4 = format_leg(FMT_Q4, 2000)
+            q4 = format_leg(FMT_Q4, 2000, "q4")
         except Exception as e:
             q4 = {"error": repr(e)}
 
@@ -538,6 +569,13 @@ def run_ours(args):
         del h_a, h_b, d_a, d_b
     except Exception as e:
         link = {"error": repr(e)}
+
+    if dumping:
+        total = sum(a.nbytes for a in dumps.values())
+        assert total <= DUMP_LIMIT_BYTES, total
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumps.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     per_rank = gather_objects({**placement, "e2e_ms_per_step": my_e2e_ms,
                                "e2e_GBps": e2e_payload / (my_e2e_ms * 1e-3) / 1e9})
@@ -597,13 +635,19 @@ def run_ours(args):
 
 
 def main():
+    sys.dont_write_bytecode = True   # the project modules imported below are in a tree bench.py leaves as it was
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-fp8", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a seeded sample of what every timed leg computed in its last "
+                         "step as DIR/<name>.npy (float32 / float64, ~40 MiB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

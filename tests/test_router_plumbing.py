@@ -1,13 +1,13 @@
 """BASELINE.json configs[0] and the router half of configs[3], with the UNMODIFIED reference router
-(/root/reference/src/vllm_router) — plumbing only, no GPU:
+(production-stack's src/vllm_router, installed into oracle/_ref by `make -C oracle ref`) — plumbing only, no GPU:
 
 * round-robin across 2 mock OpenAI backends, 100 synthetic /v1/completions -> 100 x 200, 50/50,
-  strictly alternating (the criterion of /root/reference/tests/e2e/test-routing.py:279-285);
+  strictly alternating (the criterion of the reference's tests/e2e/test-routing.py:279-285);
 * kv-aware routing: the router imports `lmcache.v1.cache_controller` from this repo's compat shim,
   workers register over ZMQ, and a prompt whose KV chunks sit in one instance's pool is routed to
   that instance (src/vllm_router/routers/routing_logic.py:332-428).
 
-Skipped where the reference tree is absent (e.g. the GPU box): nothing is copied from it.
+Skipped where oracle/_ref was not built: nothing of the reference is part of the repository.
 """
 import json
 import os
@@ -22,11 +22,9 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_SRC = "/root/reference/src"
-if not os.path.isdir(os.path.join(REF_SRC, "vllm_router")):
-    REF_SRC = os.path.join(ROOT, "baseline", "_ref")   # offline pip install of the same, unmodified (build())
+REF_SRC = os.path.join(ROOT, "oracle", "_ref")   # offline pip install of the reference, unmodified
 pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF_SRC, "vllm_router")),
-                                reason="reference router not present on this machine")
+                                reason="no reference install in oracle/_ref (make -C oracle ref)")
 
 
 def free_port(host="127.0.0.1"):
@@ -201,8 +199,6 @@ def test_reference_router_unit_tests_pass_on_top_of_the_stubs():
     router's behaviour: the reference's OWN unit tests of session routing (stickiness, minimal movement on
     add/remove of an endpoint) and round-robin routing pass with them (`@pytest.mark.asyncio` tests run by
     tests/stubs/pytest_asyncio_shim.py; pytest-asyncio is absent too)."""
-    if not REF_SRC.startswith("/root/reference"):
-        pytest.skip("the reference's test files are only in the reference tree")
     env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "tests", "stubs"), REF_SRC]))
     out = subprocess.run([sys.executable, "-m", "pytest", "-p", "pytest_asyncio_shim", "-p", "no:cacheprovider", "-q",
                           os.path.join(REF_SRC, "tests", "test_session_router.py"),

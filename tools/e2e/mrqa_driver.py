@@ -1,7 +1,7 @@
 """Multi-round-QA workload driver — a restatement (not a copy) of the reference harness
-benchmarks/multi-round-qa/multi-round-qa.py for the GPU box, where /root/reference does not exist.
-Where the reference tree is available (this build container) tests/test_e2e_tooling.py runs the
-unmodified harness and this driver against a recording mock backend and requires byte-identical
+benchmarks/multi-round-qa/multi-round-qa.py, for machines without a reference install.  What the
+unmodified harness sent to a recording mock backend is stored under tests/golden/;
+tests/test_e2e_tooling.py runs this driver against the same mock and requires byte-identical
 `messages`, max_tokens, stream flag and x-user-id header for every (session, turn) they share (the
 harness's first `num_users` sessions start mid-conversation, a ramp-up this driver does not imitate).
 The traffic shape:

@@ -54,13 +54,10 @@ def connector_args(mode: str, cpu_gb: float):
 
 
 def harness_path() -> str | None:
-    """The UNMODIFIED benchmarks/multi-round-qa/multi-round-qa.py: in the reference tree, or — on the GPU box —
-    the byte-identical copy `__graft_entry__.build()` placed in the git-ignored baseline/_ref."""
-    for p in ("/root/reference/benchmarks/multi-round-qa/multi-round-qa.py",
-              os.path.join(ROOT, "baseline", "_ref", "benchmarks", "multi-round-qa", "multi-round-qa.py")):
-        if os.path.exists(p):
-            return p
-    return None
+    """The UNMODIFIED benchmarks/multi-round-qa/multi-round-qa.py: the byte-identical copy `make -C oracle ref`
+    placed in the git-ignored oracle/_ref."""
+    p = os.path.join(ROOT, "oracle", "_ref", "benchmarks", "multi-round-qa", "multi-round-qa.py")
+    return p if os.path.exists(p) else None
 
 
 def run_harness(base_url: str, model: str, a, out_csv: str, seconds: float) -> dict:
@@ -126,7 +123,7 @@ def main():
     ap.add_argument("--harness-time", type=float, default=60.0)
     args = ap.parse_args()
     if args.harness and harness_path() is None:
-        raise SystemExit("--harness: the reference harness is neither under /root/reference nor in baseline/_ref")
+        raise SystemExit("--harness: the reference harness is not in oracle/_ref (make -C oracle ref)")
     args.log_dir = os.path.abspath(args.log_dir)     # the harness runs with another cwd
     os.makedirs(args.log_dir, exist_ok=True)
     subprocess.run([sys.executable, os.path.join(HERE, "make_model.py"), args.model_dir, "--layers", str(args.layers),

@@ -4,9 +4,8 @@ scaled to the GPUs given): N `vllm serve` replicas, one per GPU, every one with 
 `python -m vllm_router.app --service-discovery static --routing-logic <roundrobin|session|prefixaware|kvaware>`
 (pattern: /root/reference/tests/e2e/stress-test.sh:183-190), driven by tools/e2e/mrqa_driver.py.
 
-The router is the reference's own code: imported from /root/reference/src where that exists (the
-build container) or from baseline/_ref (an offline `pip install --target` of the reference, made by
-`__graft_entry__.build()`, git-ignored, shipped to the GPU box) — never from this repo.
+The router is the reference's own code: imported from oracle/_ref (an offline `pip install --target` of a
+production-stack checkout, made by `make -C oracle ref`, git-ignored) — never from this repo.
 
 Modes:
   none       no connector            -> every turn re-prefills its whole context on whichever replica it lands
@@ -54,10 +53,10 @@ MODEL = "synth-llama3-8b"
 
 
 def router_path() -> str:
-    for p in ("/root/reference/src", os.path.join(ROOT, "baseline", "_ref")):
-        if os.path.isdir(os.path.join(p, "vllm_router")):
-            return p
-    raise SystemExit("reference router not found: run `python __graft_entry__.py build` where /root/reference exists")
+    p = os.path.join(ROOT, "oracle", "_ref")
+    if os.path.isdir(os.path.join(p, "vllm_router")):
+        return p
+    raise SystemExit("reference router not found: run `make -C oracle ref REFERENCE=<production-stack checkout>`")
 
 
 def replica_env(mode: str, gpu: int, cpu_gb: float, pool_tag: str) -> tuple[dict, list[str]]:
